@@ -2,6 +2,7 @@
 """bench.py -- BASELINE.json's metric on BASELINE.json's configs.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config fwd|fwdbwd|cascade|train8]
+                    [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W      (one rank per GPU)
 
 --config fwd (default, BASELINE configs[1], the judged line): image-pairs/sec of the MaskFlownet-S forward at 1024x448,
@@ -245,6 +246,23 @@ def timed(c, fn, K, sync_extra=None):
     return c.mdist.max_over_ranks(e0.elapsed_time(e1), c.dev)
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(directory, arrays):
+    """Write {name: float32 array} as <directory>/<name>.npy: what the timed path returned in its last step, for comparing
+    two builds output for output (the inputs and weights are seeded, so equal arguments give equal inputs).  Compare with a
+    tolerance: the centralize mean and the warp backward's input / weight gradients are atomic fp32 sums, and cuDNN picks
+    its backward algorithms at run time, so repeated runs of one build differ in the last bits."""
+    import numpy as np
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"bench.py: --dump-outputs would write {total} bytes (limit {DUMP_LIMIT_BYTES})")
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
+
+
 def base_line(metric, value, K, Wm, ms_total, world, config):
     return {"metric": metric, "value": round(value, 3), "unit": "pairs/s", "n_gpus": world, "steps": K, "warmup": Wm,
             "ms_per_step": round(ms_total / K, 4), "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
@@ -276,8 +294,10 @@ def bench_fwd(args, K, Wm):
     def step_eager():
         return network.predict_flow(model, a_d, b_d)
 
+    last = {}
+
     def step_graph():
-        return graph_pred(a_d, b_d)
+        last["flow"] = graph_pred(a_d, b_d)
 
     it = [0]
 
@@ -298,6 +318,7 @@ def bench_fwd(args, K, Wm):
         ms_total = timed(c, step_graph, K)
         torch.cuda.profiler.stop()
         clocks = sampler.finish()
+        outputs = {k: v.cpu().numpy() for k, v in last.items()}    # the graph's output buffer: later replays overwrite it
         # ---- e2e: host buffers through the serving API; copies inside the timed region ----
         ms_e2e = timed(c, step_e2e, K, sync_extra=lambda: (torch.cuda.current_stream().wait_stream(serve.d2h),
                                                            torch.cuda.current_stream().wait_stream(serve.h2d)))
@@ -403,6 +424,8 @@ def bench_fwd(args, K, Wm):
             line["cpu_baseline"] = {"value": None, "unit": "pairs/s", "cores": host_threads, "kind": "port",
                                     "sample": f"failed: {e}"}
     if c.rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line), flush=True)
     if c.world > 1:
         torch.distributed.destroy_process_group()
@@ -477,8 +500,10 @@ def bench_other(args, K, Wm):
         d2h = loss_h.numel() * 4
         extra["grad_bucket_mb"] = round(bucket.numel * 4 / 1e6, 1)
 
+    last = {}
+
     def step_resident():
-        step(a_d, b_d, flow_d)
+        last["flow" if cfg == "cascade" else "per_sample_loss"] = step(a_d, b_d, flow_d)
 
     def step_e2e():
         x1, x2 = a_h.to(c.dev, non_blocking=True), b_h.to(c.dev, non_blocking=True)
@@ -496,6 +521,9 @@ def bench_other(args, K, Wm):
     ms_total = timed(c, step_resident, K)
     torch.cuda.profiler.stop()
     launches = _lib.launch_count() - n0
+    outputs = {k: v.cpu().numpy() for k, v in last.items()}
+    if cfg != "cascade":
+        outputs["grad"] = bucket.flat.cpu().numpy()       # every p.grad is a view into the bucket (parameter order)
     ar_ms = sum(x.elapsed_time(y) for x, y in t_ar) / len(t_ar) if t_ar else None
     ms_e2e = timed(c, step_e2e, K)
     clocks = sampler.finish()
@@ -523,6 +551,8 @@ def bench_other(args, K, Wm):
         extra["nccl_ranks"] = c.world
     line.update(extra)
     if c.rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line), flush=True)
     if c.world > 1:
         torch.distributed.destroy_process_group()
@@ -540,12 +570,18 @@ def main():
     ap.add_argument("--train-tc-forward", type=int, default=-1,
                     help="fwdbwd / train8: 1 = the 3x3 convolutions' forward on the tcgen05 kernel (cuDNN backward), 0 = cuDNN "
                          "both ways, -1 = the model's default")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the timed path returned in its last step as DIR/<name>.npy "
+                         "(float32; rank 0): fwd and cascade the flow; fwdbwd and train8 the per-sample loss and the "
+                         "gradient of every parameter, flattened in parameter order (train8: after the all-reduce)")
     args = ap.parse_args()
     K, Wm = args.steps, max(args.warmup, 0)
     rank = int(os.environ.get("RANK", "0"))
     host_threads = usable_host_threads()
 
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the GPU path's outputs: it needs --impl ours")
         if rank != 0:
             return
         val, sec, used = cpu_arm(max(1, K), max(1, min(Wm, 1)), host_threads)

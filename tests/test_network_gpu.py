@@ -1,6 +1,5 @@
 """GPU tests of the product model graph: against the golden fixture from the reference's own graph, against the oracle
-network on fresh inputs, the cascade, a training step, and the reference model file running unchanged on the CUDA
-operators through the mx shim (when the reference tree is present)."""
+network on fresh inputs, the cascade, a training step, and the mx shim's operator call style on the CUDA operators."""
 import os
 import sys
 
@@ -10,7 +9,7 @@ import torch
 
 pytestmark = pytest.mark.gpu
 
-from maskflownet_b200 import _lib, mx, network, ops  # noqa: E402
+from maskflownet_b200 import _lib, network, ops  # noqa: E402
 from oracle import network_ref  # noqa: E402
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -123,18 +122,6 @@ def test_training_step_gradients_flow_through_cuda_backward():
     for name in ("deform5.weight", "deform2.bias", "conv2f.weight", "conv1a.weight", "pred_mask3.weight"):
         g = dict(model.named_parameters())[name].grad
         assert g is not None and torch.isfinite(g).all() and g.abs().max().item() > 0, name
-
-
-@pytest.mark.skipif(not os.path.isdir("/root/reference/network"), reason="reference tree not present on this box")
-def test_reference_file_runs_unchanged_on_cuda_operators():
-    ref = mx.load_reference_network("/root/reference")
-    from maskflownet_b200.mx import ndarray as F
-    net = ref.MaskFlownet_S(config=mx.Reader({}))
-    net.initialize(seed=0, device="cuda")
-    a1, a2 = seeded_images()
-    with torch.no_grad():
-        preds, occ, srcs = net(F.NDArray(a1.cuda()), F.NDArray(a2.cuda()))
-    assert preds[-1].shape == (1, 2, 16, 32)
 
 
 def test_shim_operator_call_style_on_cuda():

@@ -10,6 +10,7 @@ against the oracle.
 import ctypes
 import os
 import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -19,6 +20,7 @@ from oracle import augment_ref
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 FIX = os.path.join(HERE, "golden", "aug_ref_graph.npz")
+sys.path.insert(0, os.path.join(HERE, "golden"))
 GEO_NAMES = ["rotation", "aspect_ratio", "scale", "tx_unit", "tx_range", "ty_unit", "ty_range", "rel_rotation", "rel_scale",
              "rel_translation"]
 
@@ -576,12 +578,13 @@ def test_pipeline_host_plumbing_on_cpu(monkeypatch):
         pipe.fix_head()                      # only the cascade has a head to freeze
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/weights/dbbSep30-1206_1000000.params"), reason="shipped checkpoints not on this box")
-def test_pipeline_load_head_and_fix_head_on_cpu():
+def test_pipeline_load_head_and_fix_head_on_cpu(tmp_path):
     """main.py:133-139: a MaskFlownet-S checkpoint goes into the cascade's head (load_head), which is then frozen (fix_head);
-    the trainer only keeps the cascade's own parameters."""
+    the trainer only keeps the cascade's own parameters.  The checkpoint is the shipped one's byte layout, rebuilt from
+    tests/golden/checkpoint_layout.npz."""
+    from make_golden_checkpoints import CHECKPOINT_S, rebuild_checkpoint
     from maskflownet_b200 import params as mparams, pipeline
-    ck = "/root/reference/weights/dbbSep30-1206_1000000.params"
+    ck = rebuild_checkpoint(CHECKPOINT_S, tmp_path)
     pipe = pipeline.PipelineFlownet(device="cpu", network_class="MaskFlownet")
     pipe.load_head(ck)
     raw = mparams.read_params(ck)
@@ -597,8 +600,6 @@ def test_pipeline_load_head_and_fix_head_on_cpu():
 
 
 @pytest.mark.gpu
-@pytest.mark.xfail(strict=False, reason="first run on hardware happens at round end: the round's GPU allowance was spent before "
-                                        "pipeline.py was written (host plumbing is covered by the CPU test above)")
 def test_pipeline_train_validate_predict_on_gpu():
     from maskflownet_b200 import augment, pipeline
     rng = np.random.default_rng(1)
